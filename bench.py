@@ -358,6 +358,25 @@ class LJpegBatch:
         return ok
 
 
+def dump_outputs(torch, path, batch, d_out, plan, nsample=8 << 20):
+    """What the last step of the timed path handed its caller, as .npy files under `path`: every
+    frame's pixel sum (exact in float64), a fixed sample of pixels (seed 0: the same positions
+    in every run with the same arguments) and every segment's (status, consumed)."""
+    os.makedirs(path, exist_ok=True)
+    st = plan.results(check=False)
+    px = d_out[:batch.out_bytes].view(torch.int16).view(batch.n, batch.ob // 2)
+    sums = np.array([float((px[k, :H * batch.out_pitch // 2].view(H, -1)[:, :W].to(torch.int64) & 0xFFFF)
+                           .sum().item()) for k in range(batch.n)], dtype=np.float64)
+    flat = np.sort(np.random.default_rng(0).integers(0, batch.n * H * W, nsample))
+    f, y, x = flat // (H * W), flat % (H * W) // W, flat % W
+    at = torch.from_numpy(f * (batch.ob // 2) + y * (batch.out_pitch // 2) + x).cuda()
+    sample = (px.view(-1)[at].to(torch.int32) & 0xFFFF).to(torch.float32).cpu().numpy()
+    np.save(os.path.join(path, "frame_pixel_sums.npy"), sums)
+    np.save(os.path.join(path, "pixel_sample.npy"), sample)
+    np.save(os.path.join(path, "segment_status.npy"), np.array([s for s, _ in st], dtype=np.float64))
+    np.save(os.path.join(path, "segment_consumed.npy"), np.array([c for _, c in st], dtype=np.float64))
+
+
 def C_sizeof_scan(rs):
     import ctypes
     return ctypes.sizeof(rs.LJpegScan)
@@ -578,6 +597,9 @@ def main():
     ap.add_argument("--unvalidated", action="store_true",
                     help="with --all-legs: include the post-decode kernels K9-K12 and Panasonic V4")
     ap.add_argument("--skip-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0's frames) "
+                         "as DIR/<name>.npy, about 35 MB")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -639,6 +661,8 @@ def main():
         l0 = ctx.launches
         ms = time_steps(torch, run, args.steps, args.warmup, dist)
         launches = ctx.launches - l0 - args.warmup * plan.launches
+        if args.dump_outputs and rank == 0:
+            dump_outputs(torch, args.dump_outputs, batch, d_out, plan)
         sus_n, sus_ms = 0, 0.0
         t_pre = time.perf_counter()
         while time.perf_counter() - t_pre < args.sustain_s:

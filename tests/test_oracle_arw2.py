@@ -7,7 +7,7 @@ import pytest
 import oracle
 from oracle import port, synth
 
-pytestmark = pytest.mark.skipif(not oracle.HAVE_REF, reason="reference build not available")
+pytestmark = pytest.mark.skipif(not oracle.ref.available(), reason="no reference answers (oracle/_ref or tests/golden/ref_calls)")
 
 
 @pytest.mark.parametrize("w,h", [(32, 1), (64, 5), (320, 33), (9600, 2)])

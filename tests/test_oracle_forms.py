@@ -10,7 +10,7 @@ import oracle
 from oracle import port, synth
 
 ref = oracle.ref
-pytestmark = pytest.mark.skipif(not oracle.HAVE_REF, reason="oracle/_ref/libref.so not built")
+pytestmark = pytest.mark.skipif(not oracle.ref.available(), reason="no reference answers (oracle/_ref or tests/golden/ref_calls)")
 
 
 def both(data, mk_img, w, cpp, crop, pitch, bps, order, form, curve=None, dither=False):

@@ -8,7 +8,7 @@ import pytest
 import oracle
 from oracle import port, synth
 
-pytestmark = pytest.mark.skipif(not oracle.HAVE_REF, reason="reference build not available")
+pytestmark = pytest.mark.skipif(not oracle.ref.available(), reason="no reference answers (oracle/_ref or tests/golden/ref_calls)")
 
 NCPL, VALS = synth.DEFAULT_NCPL, synth.DEFAULT_VALUES
 

@@ -8,7 +8,7 @@ import oracle
 from oracle import port, synth
 
 ref = oracle.ref
-pytestmark = pytest.mark.skipif(not oracle.HAVE_REF, reason="oracle/_ref/libref.so not built")
+pytestmark = pytest.mark.skipif(not oracle.ref.available(), reason="no reference answers (oracle/_ref or tests/golden/ref_calls)")
 
 
 def both(img_shape, w, data, meta=None, meta_be=True):

@@ -7,7 +7,7 @@ import pytest
 import oracle
 from oracle import port, synth
 
-pytestmark = pytest.mark.skipif(not oracle.HAVE_REF, reason="reference build not available")
+pytestmark = pytest.mark.skipif(not oracle.ref.available(), reason="no reference answers (oracle/_ref or tests/golden/ref_calls)")
 
 
 @pytest.mark.parametrize("w,h,wild", [(8, 1, False), (70, 9, False), (258, 33, True), (1000, 12, False)])
